@@ -10,9 +10,9 @@ contiguous blocks over the N GPUs; one "step" = every rank fetches one batch of 
 indices are seeded per rank and per step.
 
 Printed JSON (one line, rank 0):
-  value      aggregate GB/s over all ranks, indices and output resident in HBM. The K-step block (K back-to-back async
-             launches between two CUDA events on the launching stream, barrier + synchronize on both sides, max over
-             ranks) is repeated R times; value comes from the MEDIAN block, p10/p50/p90 of ms_per_step are printed too
+  value      aggregate GB/s over all ranks, indices and output resident in HBM: one block of exactly K back-to-back
+             async launches between two CUDA events on the launching stream, barrier + synchronize on both sides, max
+             over ranks
   verified_rows  rows of the LAST timed batch of every rank regenerated and compared on the device (all of them, at
              every N), with the number of requests every owner served
   e2e        same metric through the host-facing call: pinned HOST index arrays in, pinned HOST buffer out,
@@ -56,9 +56,10 @@ CFG5_SIZES = (1 << 10, 4 << 10, 16 << 10, 64 << 10, 256 << 10, 1 << 20, 4 << 20,
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=200, help="timed launches of the headline, in one block")
     ap.add_argument("--warmup", type=int, default=5)
-    ap.add_argument("--repeats", type=int, default=10, help="how many times the K-step timed block is repeated")
+    ap.add_argument("--repeats", type=int, default=10,
+                    help="how many times the timed block of each extra config is repeated (the headline times --steps steps)")
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--batch", type=int, default=65536, help="samples per rank per step")
     ap.add_argument("--samples", type=int, default=TOTAL_SAMPLES, help="total samples (default: the full config)")
@@ -73,6 +74,10 @@ def parse():
                          "of the default run)")
     ap.add_argument("--configs", default="cfg3,cfg4,cfg5,cfg1,persample,ingest,prefetch")
     ap.add_argument("--config-scale", type=float, default=1.0, help="shrink the stores of the extra configs (tests)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write a fixed seeded sample of the rows the headline's last timed step "
+                         "fetched to DIR/batch_rows_rank<r>.npy (the rows' 32-bit words as float64; 4096 rows, 32 MiB, "
+                         "over all ranks together), to compare two builds output for output")
     return ap.parse_args()
 
 
@@ -226,6 +231,12 @@ def calibrate_threads(cpu_samples, cpu_batch):
 _CAL = {}
 
 
+def reference_world():
+    """-> (kind, world class): the compiled reference when oracle/_ref is built, else the oracle's C port"""
+    from oracle import oracle as O
+    return ("reference", O.RefWorld) if O.have_ref() else ("port", O.PortWorld)
+
+
 def cpu_reference_run(cpu_samples, cpu_batch, steps, warmup, nthreads=None):
     """The reference's own get() path on the host cores: the UNMODIFIED DDStore (method 0) compiled against the
     MPI thread-rank shim when oracle/_ref is built, else the oracle's C port. One rank-thread per core,
@@ -246,40 +257,20 @@ def cpu_reference_run(cpu_samples, cpu_batch, steps, warmup, nthreads=None):
     outs = [np.empty(cpu_batch * ROW_BYTES, np.uint8) for _ in range(P)]
     counts = [np.ones(cpu_batch, np.int64) for _ in range(P)]
     times = []
-    if O.have_ref():
-        kind = "reference"
-        w = O.RefWorld(P)
-        w.add("x", shards)
-        for it in range(warmup + steps):
-            starts = [rng.integers(0, total, size=cpu_batch) for rng in rngs]
-            ns = w.get_loop_all("x", starts, counts, outs)
-            if ns < 0:
-                raise RuntimeError("reference get() failed: " + w.err())
-            if it >= warmup:
-                times.append(ns * 1e-9)
-        # parity spot check of the timed path against the generator
-        exp = co.synth_rows(SEED, int(starts[0][-1]), 1, DISP, np.float32)
-        assert outs[0][-ROW_BYTES:].tobytes() == exp.tobytes()
-        w.close()
-    else:
-        kind = "port"
-        import ctypes as C
-        bases = (C.c_void_p * P)(*[s.ctypes.data for s in shards])
-        ll = O.np_lenlist([per] * P)
-        LP = C.POINTER(C.c_long)
-
-        def one(r, starts):
-            co.L.orc_get_batch(bases, ll.ctypes.data_as(LP), P, DISP, 4, 4, starts.ctypes.data_as(LP),
-                               counts[r].ctypes.data_as(LP), cpu_batch, outs[r].ctypes.data, None, None)
-
-        for it in range(warmup + steps):
-            starts = [np.ascontiguousarray(rng.integers(0, total, size=cpu_batch)) for rng in rngs]
-            th = [threading.Thread(target=one, args=(r, starts[r])) for r in range(P)]
-            t0 = time.perf_counter()
-            [t.start() for t in th]
-            [t.join() for t in th]
-            if it >= warmup:
-                times.append(time.perf_counter() - t0)
+    kind, World = reference_world()
+    w = World(P)
+    w.add("x", shards)
+    for it in range(warmup + steps):
+        starts = [rng.integers(0, total, size=cpu_batch) for rng in rngs]
+        ns = w.get_loop_all("x", starts, counts, outs)
+        if ns < 0:
+            raise RuntimeError("reference get() failed: " + w.err())
+        if it >= warmup:
+            times.append(ns * 1e-9)
+    # parity spot check of the timed path against the generator
+    exp = co.synth_rows(SEED, int(starts[0][-1]), 1, DISP, np.float32)
+    assert outs[0][-ROW_BYTES:].tobytes() == exp.tobytes()
+    w.close()
     step_bytes = P * cpu_batch * ROW_BYTES
     t = float(np.sum(times))
     gbs = step_bytes * len(times) / t / 1e9
@@ -297,8 +288,7 @@ def cpu_reference_configs(names, nthreads, steps=3, warmup=1):
     """The reference's get() loop (count > 1: ONE MPI_Get of count rows per request, ddstore.hpp:229-236) on the shapes of
     configs 3 / 4 / 5 / 1, bounded samples, `nthreads` rank-threads. -> {config name: {value, samples_per_s, ...}}"""
     from oracle import oracle as O
-    if not O.have_ref():
-        return {}
+    kind, World = reference_world()
     co = O.COracle()
     P = max(1, nthreads)
     out = {}
@@ -317,7 +307,7 @@ def cpu_reference_configs(names, nthreads, steps=3, warmup=1):
                 ts.append(t)
         tt = float(np.mean(ts))
         return {"value": nbytes_per_step / tt / 1e9, "unit": UNIT, "samples_per_s": nsamples_per_step / tt,
-                "ms_per_step": 1e3 * tt, "cores": P, "kind": "reference", "sample": label}
+                "ms_per_step": 1e3 * tt, "cores": P, "kind": kind, "sample": label}
 
     if "cfg3" in names:
         nsamp = 2048 * P  # ~20 KB each: ~40 MB per rank-thread
@@ -325,7 +315,7 @@ def cpu_reference_configs(names, nthreads, steps=3, warmup=1):
         per = nsamp // P
         shards = [co.synth_rows(SEED, int(sstart[r * per]), int(sstart[(r + 1) * per] - sstart[r * per]), 1, np.float32)
                   for r in range(P)]
-        w = O.RefWorld(P)
+        w = World(P)
         w.add("x", shards)
         del shards
         for B in (4096, 16384):
@@ -346,7 +336,7 @@ def cpu_reference_configs(names, nthreads, steps=3, warmup=1):
         per = nsamp // P
         nf = [co.synth_rows(SEED, int(ns_[r * per]), int(ns_[(r + 1) * per] - ns_[r * per]), 16, np.float32) for r in range(P)]
         ei = [co.synth_rows(SEED + 1, int(es_[r * per]), int(es_[(r + 1) * per] - es_[r * per]), 2, np.int64) for r in range(P)]
-        w = O.RefWorld(P)
+        w = World(P)
         w.add("node_feat", nf)
         w.add("edge_index", ei)
         del nf, ei
@@ -367,7 +357,7 @@ def cpu_reference_configs(names, nthreads, steps=3, warmup=1):
             if R * rows_per * P > (8 << 30):  # bound the host memory (twice this: add() copies) and the set-up time
                 rows_per = max(4, (8 << 30) // (R * P))
             shards = [co.synth_rows(SEED, r * rows_per, rows_per, R // 4, np.float32) for r in range(P)]
-            w = O.RefWorld(P)
+            w = World(P)
             w.add("s", shards)
             del shards
             b = max(2, min(4096, (16 << 20) // R))
@@ -383,7 +373,7 @@ def cpu_reference_configs(names, nthreads, steps=3, warmup=1):
         rows = 262144
         data = [co.synth_rows(SEED, 0, rows, DISP, np.float32)]
         lab = [co.synth_rows(SEED + 2, 0, rows, 1, np.int32)]
-        w = O.RefWorld(1)
+        w = World(1)
         w.add("d", data)
         w.add("l", lab)
         b = 65536
@@ -846,13 +836,32 @@ def bench_prefetch(ctx, sc):
     return e
 
 
+DUMP_ROWS = 4096  # rows dumped over all ranks together: 4096 rows x 1024 words x 8 B = 32 MiB as float64
+
+
+def sample_batch(packed, B, N):
+    """DUMP_ROWS // N of the B packed rows one rank received, at positions drawn from a fixed seed, copied to the host
+    as uint32 [rows, DISP]"""
+    import torch
+    sel = np.sort(np.random.default_rng(SEED).choice(B, size=min(B, max(1, DUMP_ROWS // N)), replace=False))
+    return packed.view(torch.int32).view(B, DISP)[torch.from_numpy(sel).to(packed.device)].cpu().numpy().view(np.uint32)
+
+
+def dump_batch(dirname, rank, rows):
+    """DIR/batch_rows_rank<r>.npy: float64 [rows, DISP], each row's 32-bit words as unsigned integers. The payload is raw
+    bit patterns (NaN, Inf among them as float32); every uint32 is exact and finite in float64, so the file carries the
+    bytes bit for bit"""
+    os.makedirs(dirname, exist_ok=True)
+    np.save(os.path.join(dirname, f"batch_rows_rank{rank}.npy"), rows.astype(np.float64))
+
+
 def run_ours(args):
     import torch
     from ddstore_b200 import PyDDStore, _capi
 
     ctx = Ctx(args)
     N, rank, local, dev, stream = ctx.N, ctx.rank, ctx.local, ctx.dev, ctx.stream
-    K, W, B, R = args.steps, max(args.warmup, 3), args.batch, max(1, args.repeats)
+    K, W, B = args.steps, max(args.warmup, 3), args.batch
     total = args.samples
     nrows = ctx.share(total)
 
@@ -881,17 +890,17 @@ def run_ours(args):
         sampler.start()
         time.sleep(0.3)
     launches0 = _capi.lib().dds_kernel_launches()
-    ms_blocks = ctx.timed_blocks(store, lambda i: store.get_batch("x", idx_dev[i % nsets], out=outs[i & 1], count=1, stream=stream,
-                                                                  wait=False, overlap=True), K, W, R)
-    launches = (_capi.lib().dds_kernel_launches() - launches0) * K // (W + R * K)  # kernels per K-step block
+    ms_step = ctx.timed_blocks(store, lambda i: store.get_batch("x", idx_dev[i % nsets], out=outs[i & 1], count=1, stream=stream,
+                                                                wait=False, overlap=True), K, W, 1)[0]
+    launches = (_capi.lib().dds_kernel_launches() - launches0) * K // (W + K)  # kernels per K-step block
     clocks = sampler.stop() if rank == 0 else None
     # every row of the last two timed batches of every rank, regenerated and compared on the device
-    last = W + R * K - 1
+    last = W + K - 1
     ver = [verify_entry(ctx, store, "x", outs[i & 1], idx_dev[i % nsets], None, 1, None, SEED, B) for i in (last - 1, last)]
+    dumped = sample_batch(outs[last & 1], B, N) if args.dump_outputs else None  # (the buffer is reused below)
     owners_hit = min(v[2] for v in ver)
     if B >= 64 * N:
         assert owners_hit == N, f"bench: only {owners_hit} of {N} owners served requests"
-    ms_step = float(np.median(ms_blocks))
     value = N * step_bytes / (ms_step * 1e-3) / 1e9
 
     # second pass, K steps, one CUDA-event pair around every launch: the kernel's own duration serialised
@@ -919,13 +928,13 @@ def run_ours(args):
         def push_step(i):
             last_view[i & 1] = store.get_batch_push("x", idx_dev[i % nsets], count=1, stream=stream)
 
-        ms_push = ctx.timed_blocks(store, push_step, K, W, R)
+        ms_p = ctx.timed_blocks(store, push_step, K, W, 1)[0]
         # (the window's buffers alternate with the store's own step counter; verify what the last two steps returned)
-        lastp = W + R * K - 1
+        lastp = W + K - 1
         pver = [verify_entry(ctx, store, "x", last_view[i & 1], idx_dev[i % nsets], None, 1, None, SEED, B) for i in (lastp - 1, lastp)]
-        ms_p = float(np.median(ms_push))
+        dumped_push = sample_batch(last_view[lastp & 1], B, N) if args.dump_outputs else None
         push = {"value": N * step_bytes / (ms_p * 1e-3) / 1e9, "unit": UNIT, "ms_per_step": ms_p,
-                "ms_per_step_p10_p50_p90": pct(ms_push), "roofline": ctx.roofline(step_bytes, ms_p),
+                "roofline": ctx.roofline(step_bytes, ms_p),
                 "verified_rows": sum(v[0] for v in pver), "mismatches": sum(v[1] for v in pver),
                 "path": "dds_get_batch_push: every rank publishes its start rows, every owner TMA-stores the rows it owns into "
                         "the requesters' peer-mapped windows, arrival signalled with system-scope words; one launch per rank "
@@ -1012,22 +1021,24 @@ def run_ours(args):
     pull = None
     if push and push["value"] > value:
         # the headline is the faster of the two ways a DDP loader can fetch its batch; the other one is kept beside it
-        pull = {"value": value, "ms_per_step": ms_step, "ms_per_step_p10_p50_p90": pct(ms_blocks), "roofline": dict(roofline)}
-        value, ms_step, ms_blocks = push["value"], push["ms_per_step"], ms_push
+        pull = {"value": value, "ms_per_step": ms_step, "roofline": dict(roofline)}
+        value, ms_step, dumped = push["value"], push["ms_per_step"], dumped_push
         roofline.update(push["roofline"])
         roofline["per_launch_ms"] = ms_step
         fetch_mode = "collective owner-push (dds_get_batch_push)"
+    if args.dump_outputs:  # the rows of the last timed step of the path the headline reports
+        dump_batch(args.dump_outputs, rank, dumped)
     if rank == 0:
         line = {"metric": METRIC, "value": value, "unit": UNIT, "n_gpus": N, "steps": K, "warmup": W,
-                "ms_per_step": ms_step, "ms_per_step_p10_p50_p90": pct(ms_blocks), "repeats": R,
+                "ms_per_step": ms_step,
                 "fetch_mode": fetch_mode, "pull": pull, "push": push,
                 "serialized_ms_per_step": float(np.median(ser_blocks)),
                 "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
                 "dtype": "u8", "data": "synthetic",
                 "config": workload_config(N, total, B),
-                "method": {"queue": "K independent batches per block queued asynchronously on one stream with DDS_OVERLAP into "
-                                    "two alternating output buffers (double-buffered prefetch; the kernel enforces that batch "
-                                    "k+2 writes nothing before batch k retired); R blocks, median reported",
+                "method": {"queue": "K independent batches in one timed block queued asynchronously on one stream with DDS_OVERLAP "
+                                    "into two alternating output buffers (double-buffered prefetch; the kernel enforces that "
+                                    "batch k+2 writes nothing before batch k retired)",
                            "mapping": "VMM peer mappings (fd passing), no NCCL in the data path",
                            "gather_geometry": {"ctas": geom[0].value, "warps_per_cta": geom[1].value,
                                                "stages": geom[2].value, "chunk_bytes": geom[3].value,

@@ -3,6 +3,7 @@
 ctypes loaders for
   * liboracle.so                (oracle/ddstore_oracle.c, the plain-C restatement), class `COracle`
   * _ref/libddstore_ref.so      (the UNMODIFIED reference compiled against oracle/mpi_shim), class `RefWorld`
+    (`PortWorld` runs the same timed loops on liboracle.so where _ref is not built)
 and an independent NumPy restatement (`np_*` functions) used to cross-check both.
 
 Reference lines followed by the NumPy restatement:
@@ -15,6 +16,8 @@ Reference lines followed by the NumPy restatement:
 import ctypes as C
 import os
 import subprocess
+import threading
+import time
 
 import numpy as np
 
@@ -171,6 +174,52 @@ class COracle:
         out = np.zeros((nrows, disp), dtype)
         self.L.orc_synth_rows(seed, first_global_row, nrows, disp, dtype.itemsize, out.ctypes.data)
         return out
+
+
+class PortWorld:
+    """`size` thread-ranks of the C restatement with the part of RefWorld's surface a timed get() loop needs (add,
+    get_loop_all): the stand-in for the reference where oracle/_ref is not built."""
+
+    def __init__(self, size):
+        self.co, self.size, self.vars, self._err = COracle(), size, {}, ""
+
+    def close(self):
+        self.vars.clear()
+
+    def err(self):
+        return self._err
+
+    def add(self, name, shards):
+        shards = [np.ascontiguousarray(s) for s in shards]
+        self.vars[name] = (shards, np_lenlist([s.shape[0] for s in shards]))
+
+    def get_loop_all(self, name, starts_per_rank, counts_per_rank, outs):
+        """concurrent loops, one thread per rank, each into its packed buffer; returns the wall ns of the slowest
+        rank, or -1 with err() set when a request fails"""
+        shards, ll = self.vars[name]
+        disp = int(np.prod(shards[0].shape[1:], dtype=np.int64))
+        itemsize = shards[0].dtype.itemsize
+        bases = (C.c_void_p * len(shards))(*[s.ctypes.data for s in shards])
+        LP = C.POINTER(C.c_long)
+        st = [np.ascontiguousarray(s, dtype=np.int64) for s in starts_per_rank]
+        ct = [np.ascontiguousarray(c, dtype=np.int64) for c in counts_per_rank]
+        rcs = [0] * self.size
+
+        def one(r):
+            rcs[r] = self.co.L.orc_get_batch(bases, ll.ctypes.data_as(LP), len(shards), disp, itemsize, itemsize,
+                                             st[r].ctypes.data_as(LP), ct[r].ctypes.data_as(LP), len(st[r]),
+                                             outs[r].ctypes.data, None, None)
+
+        th = [threading.Thread(target=one, args=(r,)) for r in range(self.size)]
+        t0 = time.perf_counter()
+        [t.start() for t in th]
+        [t.join() for t in th]
+        ns = int((time.perf_counter() - t0) * 1e9)
+        bad = [rc for rc in rcs if rc]
+        if bad:
+            self._err = ERR_TEXT[bad[0]]
+            return -1
+        return ns
 
 
 # --------------------------------------------------------------------------- the real reference

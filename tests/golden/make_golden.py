@@ -1,4 +1,4 @@
-"""tests/golden/make_golden.py -- generates tests/golden/golden.json.
+"""tests/golden/make_golden.py -- generates tests/golden/golden.json and tests/golden/reference_cases.json.
 
 Runs the UNMODIFIED reference (oracle/_ref/libddstore_ref.so: /root/reference/include/ddstore.hpp
 + src/ddstore.cxx compiled verbatim against oracle/mpi_shim) on small seeded worlds and records,
@@ -18,8 +18,10 @@ import numpy as np
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.path.insert(0, ROOT)
 from oracle.oracle import RefWorld  # noqa: E402
+from tests.helpers import random_valid_requests, random_world  # noqa: E402
 
 OUT = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden.json")
+OUT_REF = os.path.join(os.path.dirname(os.path.abspath(__file__)), "reference_cases.json")
 
 
 def payload(seed, nrows, disp, dtype):
@@ -105,7 +107,105 @@ def case_demo_py(seed=20260921):
     return out
 
 
+RANDOM_WORLDS = [("float32", 1, 4), ("float32", 16, 8), ("int64", 2, 3), ("uint8", 7, 2), ("float64", 5, 1),
+                 ("int32", 3, 5), ("bool", 3, 2)]
+OUTCOME_CODES = {None: ".", "Invalid start on target": "s", "Invalid count on target": "c"}
+
+
+def case_random_world(dtype, disp, P):
+    """a seeded random world, 300 valid requests as one serial get() loop, then 400 arbitrary (mostly invalid) single
+    get() calls: their outcome (one letter of OUTCOME_CODES each) and the sha256 of the rows of the valid ones, in order"""
+    dt = np.dtype(dtype)
+    seed = 1000 + disp * 31 + P
+    rng = np.random.default_rng(seed)
+    nrows, shards = random_world(rng, P, dt, disp)
+    w = RefWorld(P)
+    w.add("v", shards)
+    it, dp, ll = w.query(0, "v")
+    starts, counts = random_valid_requests(rng, ll, 300)
+    out, bad, err, _ = w.get_batch(P - 1, "v", starts, counts)
+    assert bad == -1 and err is None
+    rec = {"dtype": dt.name, "disp": disp, "P": P, "seed": seed, "nrows": nrows, "itemsize": it, "ref_disp": dp,
+           "lenlist": ll.tolist(), "batch_nbytes": int(out.size), "batch_sha256": hashlib.sha256(out.tobytes()).hexdigest()}
+    total = int(ll[-1])
+    codes, h = [], hashlib.sha256()
+    for _ in range(400):
+        s = int(rng.integers(-5, total + 5))
+        c = int(rng.integers(0, 60))
+        buf = np.zeros((c, disp), dt)
+        try:
+            w.get(0, "v", buf, s)
+            codes.append(OUTCOME_CODES[None])
+            h.update(buf.tobytes())
+        except ValueError as e:
+            codes.append(OUTCOME_CODES[str(e)])
+    rec["probes"] = "".join(codes)
+    rec["probe_rows_sha256"] = h.hexdigest()
+    w.close()
+    return rec
+
+
+def case_init_update_fences():
+    """include/ddstore.hpp:110-195 and src/ddstore.cxx:51-77: init over 3 ranks (one empty), update 2 rows of rank 0
+    at row offset 1, read the first 4 global rows from rank 2; then the fence and disp errors"""
+    w = RefWorld(3)
+    w.init("z", [4, 0, 6], [3, 3, 3], 4, np.float32)
+    a = np.arange(6, dtype=np.float32).reshape(2, 3)
+    w.update(0, "z", a, 1)
+    got = np.full((4, 3), -1, np.float32)
+    w.get(2, "z", got, 0)
+    rec = {"P": 3, "nrows": [4, 0, 6], "disp": 3, "update": {"rank": 0, "offset": 1, "rows": a.tolist()},
+           "get": {"rank": 2, "start": 0, "count": 4, "hex": got.tobytes().hex()}, "errors": {}}
+    w.epoch_begin()
+    for key, fn, exc in (("epoch_begin_twice", w.epoch_begin, RuntimeError), ("epoch_end", w.epoch_end, None),
+                         ("epoch_end_twice", w.epoch_end, RuntimeError),
+                         ("add_disp_3_4_3", lambda: w.add("bad", [np.zeros((2, d), np.float32) for d in (3, 4, 3)]),
+                          ValueError)):
+        try:
+            fn()
+            assert exc is None, key
+        except (RuntimeError, ValueError) as e:
+            assert isinstance(e, exc), key
+            rec["errors"][key] = str(e)
+    w.close()
+    return rec
+
+
+def case_owner_lookup(n=500):
+    """src/ddstore.cxx:5-17 on seeded random row counts (1..12 ranks, 0..40 rows each, also empty ranks) and starts
+    in [-5, 500]: [nrows, start, owner]"""
+    w = RefWorld(1)
+    rng = np.random.default_rng(11)
+    out = []
+    for _ in range(n):
+        nrows = rng.integers(0, 41, size=int(rng.integers(1, 13))).tolist()
+        start = int(rng.integers(-5, 501))
+        out.append([nrows, start, w.sortedsearch(np.cumsum(nrows), start)])
+    w.close()
+    return out
+
+
+def write_reference_cases():
+    g = {"generator": "tests/golden/make_golden.py over oracle/_ref/libddstore_ref.so (reference @ 9035c779)",
+         "outcome_codes": {v: k for k, v in OUTCOME_CODES.items()},
+         "random_worlds": [case_random_world(*c) for c in RANDOM_WORLDS],
+         "init_update_fences": case_init_update_fences(),
+         "owner_lookup": case_owner_lookup()}
+    # one top-level entry (or list element) per line: small enough to review, still plain JSON
+    parts = []
+    for k, v in g.items():
+        if isinstance(v, list):
+            body = "[\n  " + ",\n  ".join(json.dumps(x, separators=(",", ":")) for x in v) + "\n ]"
+        else:
+            body = json.dumps(v, separators=(",", ":"))
+        parts.append(f" {json.dumps(k)}: {body}")
+    with open(OUT_REF, "w") as f:
+        f.write("{\n" + ",\n".join(parts) + "\n}\n")
+    print("wrote", OUT_REF, os.path.getsize(OUT_REF), "bytes")
+
+
 def main():
+    write_reference_cases()
     w = RefWorld(1)
     g = {"generator": "tests/golden/make_golden.py over oracle/_ref/libddstore_ref.so (reference @ 9035c779)",
          "sortedsearch": case_sortedsearch(w)}

@@ -13,6 +13,11 @@ def load_golden():
         return json.load(f)
 
 
+def load_reference_cases():
+    with open(os.path.join(HERE, "golden", "reference_cases.json")) as f:
+        return json.load(f)
+
+
 def golden_payload(seed, nrows, disp, dtype):
     """Same recipe as tests/golden/make_golden.py::payload (raw random bytes -> NaNs, -0, denormals...)."""
     rng = np.random.default_rng(seed)

@@ -2,15 +2,20 @@
 (oracle/oracle.py) against
   (1) the committed golden vectors the unmodified reference produced (tests/golden/golden.json),
   (2) the reference's own known answers (test/demo.cxx:20-37, test/demo.py:55-56, test/test.py:157-159),
-  (3) the verbatim-compiled reference itself (oracle/_ref) on seeded random worlds, when it is built.
+  (3) what the verbatim-compiled reference (oracle/_ref) returned on seeded random worlds
+      (tests/golden/reference_cases.json).
 CPU only."""
+import hashlib
+
 import numpy as np
 import pytest
 
 from oracle import oracle as O
-from tests.helpers import (golden_world_shards, load_golden, random_valid_requests, random_world, sha)
+from tests.helpers import (golden_world_shards, load_golden, load_reference_cases, random_valid_requests, random_world,
+                           sha)
 
 G = load_golden()
+R = load_reference_cases()
 
 
 def test_sortedsearch_golden(coracle):
@@ -108,67 +113,51 @@ def test_synth_generator_c_vs_numpy(coracle):
     assert np.isnan(f).any()  # payload deliberately contains NaN bit patterns
 
 
-@pytest.mark.skipif(not O.have_ref(), reason="oracle/_ref not built (needs /root/reference at build time)")
 @pytest.mark.parametrize("dtype,disp,P", [(np.float32, 1, 4), (np.float32, 16, 8), (np.int64, 2, 3),
                                           (np.uint8, 7, 2), (np.float64, 5, 1), (np.int32, 3, 5), (np.bool_, 3, 2)])
 def test_c_oracle_vs_compiled_reference(coracle, dtype, disp, P):
+    """against what the compiled reference returned on the same seeded world (tests/golden/reference_cases.json)"""
+    ref = next(w for w in R["random_worlds"] if (w["dtype"], w["disp"], w["P"]) == (np.dtype(dtype).name, disp, P))
     rng = np.random.default_rng(1000 + disp * 31 + P)
     nrows, shards = random_world(rng, P, dtype, disp)
-    w = O.RefWorld(P)
-    try:
-        w.add("v", shards)
-        it, dp, ll = w.query(0, "v")
-        assert ll.tolist() == O.np_lenlist(nrows).tolist() and dp == disp and it == np.dtype(dtype).itemsize
-        starts, counts = random_valid_requests(rng, ll, 300)
-        ref_out, bad, err, _ = w.get_batch(P - 1, "v", starts, counts)
-        assert bad == -1
-        c_out, c_offs, cbad, rc = coracle.get_batch(shards, starts, counts)
-        n_out, n_offs, nbad, nrc = O.np_get_batch(shards, starts, counts)
-        assert cbad == nbad == -1
-        assert ref_out.tobytes() == c_out.tobytes() == n_out.tobytes()
-        assert c_offs.tolist() == n_offs.tolist()
-        # error classification agrees request by request on arbitrary (mostly invalid) requests
-        total = int(ll[-1])
-        for _ in range(400):
-            s = int(rng.integers(-5, total + 5))
-            c = int(rng.integers(0, 60))
-            buf = np.zeros((c, disp), dtype)
-            try:
-                w.get(0, "v", buf, s)
-                ref_err = None
-            except ValueError as e:
-                ref_err = str(e)
-            t, off, rc = coracle.locate(ll, s, c)
-            assert (O.ERR_TEXT[rc] if rc else None) == ref_err
-            assert O.np_locate(ll, s, c)[2] == rc
-            if not rc:
-                o2, _, _, _ = coracle.get_batch(shards, [s], [c])
-                assert o2.tobytes() == buf.tobytes()
-    finally:
-        w.close()
+    ll = O.np_lenlist(nrows)
+    assert nrows == ref["nrows"] and ll.tolist() == ref["lenlist"]
+    assert ref["ref_disp"] == disp and ref["itemsize"] == np.dtype(dtype).itemsize
+    starts, counts = random_valid_requests(rng, ll, 300)
+    c_out, c_offs, cbad, rc = coracle.get_batch(shards, starts, counts)
+    n_out, n_offs, nbad, nrc = O.np_get_batch(shards, starts, counts)
+    assert cbad == nbad == -1
+    assert c_out.size == ref["batch_nbytes"] and sha(c_out.tobytes()) == ref["batch_sha256"]
+    assert c_out.tobytes() == n_out.tobytes()
+    assert c_offs.tolist() == n_offs.tolist()
+    # error classification agrees request by request on arbitrary (mostly invalid) requests
+    total = int(ll[-1])
+    rows = hashlib.sha256()
+    for code in ref["probes"]:
+        s = int(rng.integers(-5, total + 5))
+        c = int(rng.integers(0, 60))
+        t, off, rc = coracle.locate(ll, s, c)
+        assert (O.ERR_TEXT[rc] if rc else None) == R["outcome_codes"][code]
+        assert O.np_locate(ll, s, c)[2] == rc
+        if not rc:
+            o2, _, _, _ = coracle.get_batch(shards, [s], [c])
+            rows.update(o2.tobytes())
+    assert rows.hexdigest() == ref["probe_rows_sha256"]
 
 
-@pytest.mark.skipif(not O.have_ref(), reason="oracle/_ref not built")
-def test_reference_init_update_and_fences():
-    # include/ddstore.hpp:110-195 and src/ddstore.cxx:51-77 through the compiled reference
-    P = 3
-    w = O.RefWorld(P)
-    try:
-        w.init("z", [4, 0, 6], [3, 3, 3], 4, np.float32)
-        a = np.arange(6, dtype=np.float32).reshape(2, 3)
-        w.update(0, "z", a, 1)
-        got = np.full((4, 3), -1, np.float32)
-        w.get(2, "z", got, 0)
-        exp = np.zeros((4, 3), np.float32)
-        exp[1:3] = a
-        assert got.tobytes() == exp.tobytes()
-        w.epoch_begin()
-        with pytest.raises(RuntimeError, match="Fence already activated"):
-            w.epoch_begin()
-        w.epoch_end()
-        with pytest.raises(RuntimeError, match="Fence is not activated"):
-            w.epoch_end()
-        with pytest.raises(ValueError, match="Invalid disp"):
-            w.add("bad", [np.zeros((2, 3), np.float32), np.zeros((2, 4), np.float32), np.zeros((2, 3), np.float32)])
-    finally:
-        w.close()
+def test_reference_init_update_and_fences(coracle):
+    # include/ddstore.hpp:110-195 and src/ddstore.cxx:51-77: what the compiled reference returned, against the restatement
+    ref = R["init_update_fences"]
+    shards = [np.zeros((n, ref["disp"]), np.float32) for n in ref["nrows"]]
+    a = np.array(ref["update"]["rows"], np.float32)
+    u = ref["update"]["offset"]
+    shards[ref["update"]["rank"]][u:u + len(a)] = a
+    exp = np.zeros((4, 3), np.float32)
+    exp[1:3] = np.arange(6, dtype=np.float32).reshape(2, 3)
+    for impl in (coracle.get_batch, O.np_get_batch):
+        out, _, bad, _ = impl(shards, [ref["get"]["start"]], [ref["get"]["count"]])
+        assert bad == -1 and out.tobytes().hex() == ref["get"]["hex"] == exp.tobytes().hex()
+    assert ref["errors"] == {"epoch_begin_twice": "Fence already activated", "epoch_end_twice": "Fence is not activated",
+                             "add_disp_3_4_3": "Invalid disp"}
+    _, rc = coracle.lenlist([2, 2, 2], [3, 4, 3])
+    assert O.ERR_TEXT[rc] == ref["errors"]["add_disp_3_4_3"]
